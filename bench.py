@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload grid10x10|asia_1m|dag50]
                     [--rows R] [--impl b200|reference] [--no-extras] [--no-cpu-baseline]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic evidence rows:
 `rows` independent exact-inference queries (same query variables, same evidence
@@ -60,7 +61,32 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `extra` block (the other BASELINE configs)")
     ap.add_argument("--dump", default="", help="write per-launch timings (JSON) here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the posteriors of the last timed step to DIR/posterior.npy (float32 [Q, rows], rank "
+                         "order; beyond 64 MB a fixed, seeded sample of the rows, kept in row order)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the posteriors of the b200 arm")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array [Q, rows] as DIR/<name>.npy (float32).  When they exceed DUMP_BYTES in all,
+    the same fixed, seeded sample of rows (columns) is taken from every array."""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[1]
+    row_bytes = sum(a.shape[0] * 4 for a in arrays.values())
+    if row_bytes * n > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+        arrays = {k: a[:, keep] for k, a in arrays.items()}
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), np.ascontiguousarray(a))
 
 
 # ------------------------------------------------------------------ clocks sampling
@@ -438,9 +464,10 @@ class Timer:
         return [float(x) for x in t]
 
 
-def exact_workload(ctx, wl, rows, steps, warmup, want_profile=False, counts=None):
+def exact_workload(ctx, wl, rows, steps, warmup, want_profile=False, counts=None, keep_output=False):
     """Time one exact-inference workload on this rank's GPU (+ gather when distributed).
-    Returns a dict on rank 0 (None elsewhere): device-timed and end-to-end numbers."""
+    Returns a dict on rank 0 (None elsewhere): device-timed and end-to-end numbers, and with
+    `keep_output` the posteriors [Q, global rows] of the last device-timed step."""
     import torch
 
     from sorobn_b200 import engine, planner, sharding
@@ -483,6 +510,9 @@ def exact_workload(ctx, wl, rows, steps, warmup, want_profile=False, counts=None
     launches0 = prog.info()["launches"]
     dev_ms = tm.device_ms(device_step, steps, flush)
     launches = prog.info()["launches"] - launches0
+    posterior = None
+    if keep_output and rank == 0:  # copied before the end-to-end steps below run the rows again
+        posterior = (sp.gathered.transpose(0, 1).reshape(Q, -1) if distributed else d_out).clone()
     for _ in range(max(1, warmup // 2)):
         host_step()
     e2e_s = tm.wall_s(host_step, steps)
@@ -498,7 +528,7 @@ def exact_workload(ctx, wl, rows, steps, warmup, want_profile=False, counts=None
     ms_per_step = dev_ms / steps
     total_rows = rows * world if counts is None else int(sum(counts))
     res = {
-        "plan": plan, "prog": prog, "bn": bn, "codes_host": codes_host, "rows": rows, "flush": flush,
+        "plan": plan, "prog": prog, "bn": bn, "codes_host": codes_host, "rows": rows, "flush": flush, "posterior": posterior,
         "ms_per_step": ms_per_step, "value": total_rows / (ms_per_step * 1e-3),
         "e2e_ms_per_step": 1e3 * e2e_s / steps, "e2e_value": total_rows / (e2e_s / steps),
         "h2d": int(n_ev * rows) * world, "d2h": int(Q * rows * 4) * world, "e2e_api": e2e_api,
@@ -628,8 +658,10 @@ def run_b200(args, rank, world, local_rank):
 
     clocks = ClockSampler(local_rank)
     clocks.begin()
-    res = exact_workload(ctx, wl, rows, args.steps, args.warmup, want_profile=True)
+    res = exact_workload(ctx, wl, rows, args.steps, args.warmup, want_profile=True, keep_output=bool(args.dump_outputs))
     clocks.end()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"posterior": res["posterior"].cpu().numpy()})
     clock_summary = clocks.summary()
     clocks.close()
 

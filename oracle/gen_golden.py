@@ -158,6 +158,25 @@ def synthetic_cases(ref, synthetic, spec, n_cases, n_ev_range, seed, n_query=(1,
     return cases
 
 
+def ordered_golden(ref):
+    """The reference's operators driven in the device program's min-fill order (oracle/ref_driver.py,
+    what the CPU legs of bench.py time) on a small grid: three seeded evidence rows."""
+    from sorobn_b200 import BayesNet, planner, synthetic
+
+    kwargs = dict(rows=4, cols=4, n_states=3, seed=11)
+    spec = synthetic.grid(**kwargs)
+    net = synthetic.load(spec, BayesNet)._compiled
+    query, evs = ("g0303",), ("g0001", "g0102", "g0203", "g0300")
+    plan = planner.build_plan(net, [net.index[q] for q in query], [net.index[e] for e in evs])
+    order = [net.names[v] for v in plan.order]
+    bn = synthetic.load(spec, ref.BayesNet)
+    events = synthetic.random_events(spec, evs, 3, seed=5)
+    cases = [run_case_ordered(ref, bn, query, {v: int(events[v].iloc[b]) for v in evs}, order)
+             for b in range(len(events))]
+    return {"network": "grid4x4s3", "kind": "ordered", "generator": "grid", "kwargs": kwargs,
+            "digest": spec_digest(spec), "order": order, "cases": cases}
+
+
 def main():
     ref = import_reference()
     sys.path.insert(0, ROOT)
@@ -165,6 +184,8 @@ def main():
 
     os.makedirs(OUT, exist_ok=True)
     only_workload = "--workload-only" in sys.argv
+    with open(os.path.join(OUT, "ordered_grid4x4s3.json"), "w") as f:
+        json.dump(ordered_golden(ref), f)
 
     # ---- the reference's own example networks -------------------------------------
     for name, spec in ({} if only_workload else examples.NETWORKS).items():

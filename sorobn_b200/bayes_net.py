@@ -342,18 +342,20 @@ class BayesNet:
         return frame if n > 1 else frame.iloc[0]
 
     # ---------------------------------------------------------------------- query
-    def _plan(self, query, evidence_vars, mode, robust=False, device=None):
+    def _plan(self, query, evidence_vars, mode, robust=False, device=None, slot=0):
+        """(plan, program) for the pair on `device`, cached.  A program is not thread-safe: callers
+        that run several at once on the same device ask for distinct `slot`s."""
         with self._cache_lock:
-            return self._plan_locked(query, evidence_vars, mode, robust, device)
+            return self._plan_locked(query, evidence_vars, mode, robust, device, slot)
 
-    def _plan_locked(self, query, evidence_vars, mode, robust, device):
+    def _plan_locked(self, query, evidence_vars, mode, robust, device, slot):
         if self._compiled is None:
             self._compile()
             if self._compiled is None:
                 raise ValueError("every node needs a CPT in P before querying; call prepare()")
         net = self._compiled
         device = self.device if device is None else device
-        key = (tuple(query), tuple(evidence_vars), mode, robust, device)
+        key = (tuple(query), tuple(evidence_vars), mode, robust, device, slot)
         hit = self._engine_cache.get(key)
         if hit is None:
             for name in (*query, *evidence_vars):
@@ -533,21 +535,21 @@ class BayesNet:
             out.loc[events.index[bad]] = np.nan
         return out
 
-    def _posterior_codes(self, query, ev_vars, codes, bad, device=None):
+    def _posterior_codes(self, query, ev_vars, codes, bad, device=None, slot=0):
         """Posterior float64 [Q, n] for uint8 evidence codes [n_ev, n] on one device.  Rows the
         float32 program flags (NaN: impossible evidence, or an entry below the float32 range)
         are settled in float64 -- a few one by one with the single-event program, many as one
         batch with the batched float64 program; a row that is still NaN there is impossible."""
         n = codes.shape[1] if len(ev_vars) else len(bad)
-        _, program = self._plan(query, ev_vars, _planner.MODE_BATCHED, device=device)
+        _, program = self._plan(query, ev_vars, _planner.MODE_BATCHED, device=device, slot=slot)
         post = self._run_evicting(program, codes, n).astype(np.float64)  # [Q, n]
         suspect = np.isnan(post).any(axis=0) & ~bad
         rows = np.nonzero(suspect)[0]
         if len(rows) > 8:
-            _, robust = self._plan(query, ev_vars, _planner.MODE_BATCHED, robust=True, device=device)
+            _, robust = self._plan(query, ev_vars, _planner.MODE_BATCHED, robust=True, device=device, slot=slot)
             post[:, rows] = robust.run(np.ascontiguousarray(codes[:, rows]), len(rows))
         elif len(rows):
-            _, flat = self._plan(query, ev_vars, _planner.MODE_FLAT, device=device)
+            _, flat = self._plan(query, ev_vars, _planner.MODE_FLAT, device=device, slot=slot)
             for b in rows:
                 post[:, b] = flat.run(np.ascontiguousarray(codes[:, b:b + 1]), 1)[:, 0]
         return post
@@ -580,9 +582,11 @@ class BayesNet:
 
         n = len(bad)
         world = len(devices)
+        # a device listed k times runs k shards at once: each needs a program of its own
+        slots = [devices[:r].count(d) for r, d in enumerate(devices)]
         # programs are created up front, on this thread (the cache is not thread-safe)
-        for d in devices:
-            self._plan(query, ev_vars, _planner.MODE_BATCHED, device=d)
+        for d, s in zip(devices, slots):
+            self._plan(query, ev_vars, _planner.MODE_BATCHED, device=d, slot=s)
         plan, _ = self._plan(query, ev_vars, _planner.MODE_BATCHED, device=devices[0])
         post = np.empty((plan.Q, n), dtype=np.float64)
         errors = []
@@ -593,7 +597,7 @@ class BayesNet:
                 return
             try:
                 post[:, sl] = self._posterior_codes(query, ev_vars, np.ascontiguousarray(codes[:, sl]), bad[sl],
-                                                    device=devices[r])
+                                                    device=devices[r], slot=slots[r])
             except Exception as exc:  # surfaced on the calling thread
                 errors.append(exc)
 

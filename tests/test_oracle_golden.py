@@ -162,35 +162,30 @@ def test_oracle_gibbs_conditionals_match_reference(name):
 
 
 def test_reference_copy_driven_in_min_fill_order_matches_the_oracle():
-    """`oracle/_ref` (the reference itself, copied by oracle/build_ref.py) driven through
-    oracle/ref_driver.ordered_query -- what bench.py's CPU legs time -- gives the oracle's
-    posterior.  Skipped where the copy was not built."""
-    from oracle import build_ref, ref_driver
-    from sorobn_b200 import planner, synthetic
-
-    if not build_ref.available():
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py needs /root/reference)")
+    """The reference's own operators driven through oracle/ref_driver.ordered_query in min-fill
+    order -- what bench.py's CPU legs time -- give the oracle's posterior.  Their answers are
+    stored in tests/golden/ordered_grid4x4s3.json (oracle/gen_golden.py); where `oracle/_ref`
+    (the reference itself, copied by oracle/build_ref.py) is present, the live run must still
+    reproduce them."""
     import warnings
 
-    ref = build_ref.import_reference()
-    from sorobn_b200 import BayesNet
+    from conftest import spec_digest
+    from oracle import build_ref, ref_driver
+    from sorobn_b200 import BayesNet, synthetic
 
-    spec = synthetic.grid(4, 4, 3, seed=11)
-    ours = synthetic.load(spec, BayesNet)
-    theirs = synthetic.load(spec, ref.BayesNet)
-    net = ours._compiled
-    query, evs = ("g0303",), ("g0001", "g0102", "g0203", "g0300")
-    plan = planner.build_plan(net, [net.index[q] for q in query], [net.index[e] for e in evs])
-    order = [net.names[v] for v in plan.order]
-    dn = oracle_net(ours)
-    events = synthetic.random_events(spec, evs, 3, seed=5)
-    for b in range(len(events)):
-        event = {v: int(events[v].iloc[b]) for v in evs}
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            got = ref_driver.ordered_query(ref, theirs, query, event, order)
-        want = ve_oracle.query(dn, *query, event=event)[1].reshape(-1)
-        dense = np.zeros_like(want)
-        for k, v in got.items():
-            dense[dn.domains[query[0]].index(k)] = v
-        assert np.allclose(dense, want, rtol=1e-12, atol=0)
+    golden = load_golden("ordered_grid4x4s3")
+    spec = synthetic.grid(**golden["kwargs"])
+    assert spec_digest(spec) == golden["digest"], "synthetic generator drifted: regenerate tests/golden"
+    dn = oracle_net(synthetic.load(spec, BayesNet))
+    for case in golden["cases"]:
+        query, event = case["query"], case_event(case)
+        want = ve_oracle.query(dn, *query, event=event)[1]
+        assert np.allclose(dense_answer(case, dn.domains), want, rtol=1e-12, atol=0), case
+    if build_ref.available():
+        ref = build_ref.import_reference()
+        theirs = synthetic.load(spec, ref.BayesNet)
+        for case in golden["cases"]:
+            with warnings.catch_warnings():
+                warnings.simplefilter("ignore")
+                got = ref_driver.ordered_query(ref, theirs, case["query"], case_event(case), golden["order"])
+            assert np.allclose(got.to_numpy(), case["values"], rtol=1e-12, atol=0), case
