@@ -1016,6 +1016,7 @@ static int create_common(int device, const int32_t *words, int64_t n_words, cons
             SBN_CUDA_P(set_tiled_attrs());
             SBN_CUDA_P(sbn_chain_set_attrs());
             SBN_CUDA_P(sbn_tma_set_attrs());
+            SBN_CUDA_P(sbn_pair_set_attrs());
             done[device] = true;
         }
     }

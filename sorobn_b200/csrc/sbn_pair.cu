@@ -203,11 +203,12 @@ __global__ void __launch_bounds__(SBN_PAIR_ROWS / kV, (M1 >= SBN_PAIR_GB ? 4 : 5
     }
 }
 
-// Expanding product + contraction (SbnTripleParams): thread = one evidence row x one combination of the untouched axes.
+// Expanding product + contraction (SbnTripleParams), the body kept for A/B comparisons and for the triples the staged
+// body does not cover: thread = one evidence row x one combination of the untouched axes.
 // threadIdx.y walks the digits of a tile axis only A carries (when there is one): the warps of a CTA then work on the
 // same rows and the same entries of B and C at about the same time, and all but the first of them hit L1.
 template <int MINB>
-__global__ void __launch_bounds__(SBN_TRIPLE_THREADS, MINB) sbn_triple_kernel(const __grid_constant__ SbnTripleParams p) {
+__global__ void __launch_bounds__(SBN_TRIPLE_THREADS, MINB) sbn_triple_kernel_l1(const __grid_constant__ SbnTripleParams p) {
     constexpr int T = SBN_PAIR_T;
     sbn_pdl_entry();
     const int rblock = blockIdx.x / p.n_chunks;
@@ -278,6 +279,164 @@ __global__ void __launch_bounds__(SBN_TRIPLE_THREADS, MINB) sbn_triple_kernel(co
             for (int s = 0; s < T; ++s) __stcs(op + (static_cast<uint32_t>(row.x) * ld + z * oz + s * os), acc[z][s]);
     }
 }
+
+// packed fp32 product (mul.rn.f32x2 -> FMUL2): the first term of an inner product, as the scalar body's `a * b`
+__device__ __forceinline__ void triple_mul2(float (&r)[2], const float (&a)[2], const float (&b)[2]) {
+    unsigned long long ra, rb, rr;
+    memcpy(&ra, a, 8);
+    memcpy(&rb, b, 8);
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(rr) : "l"(ra), "l"(rb));
+    memcpy(r, &rr, 8);
+}
+
+__device__ __forceinline__ void triple_cp_async16(float *dst, const float *src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sbn_smem_u32(dst)), "l"(src) : "memory");
+}
+
+// wait until at most `n` of this thread's cp.async groups are still in flight (the count must be an immediate)
+__device__ __forceinline__ void triple_cp_async_wait(int n) {
+    if (n <= 0) asm volatile("cp.async.wait_group 0;" ::: "memory");
+    else if (n == 1) asm volatile("cp.async.wait_group 1;" ::: "memory");
+    else asm volatile("cp.async.wait_group 2;" ::: "memory");
+}
+
+// Expanding product + contraction, staged (SbnTripleParams, sbn_pair.h).  A CTA walks row blocks of R = 32 rows
+// (blockIdx.x, then every gridDim.x-th) and, per row block, p = 0 .. T-1: one "item" per (row block, p).  An item's
+// operand entries -- A[g][k][j], B[t][j][s], C[t][k][z] for this p -- are staged as 128-byte runs (32 rows, rows
+// innermost as in global memory) by cp.async into a ring of n_stages items, n_stages - 1 of them in flight while the
+// CTA computes on the oldest.
+// Thread = row pair rp (lane & 15) x slot (2 x warp + lane / 16) = (group digit g, tile t): the two half-warps read
+// the same B and C entries (one wavefront each) and two entries of A (two wavefronts).  Per item it loads its 25 B
+// entries into registers once, then per k: N[s] = sum_j A[k][j] B[j][s], acc[z][s] += C[k][z] N[s] -- the order of
+// the scalar body, on (row b, row b + 1) register pairs (FMUL2 / FFMA2): the results are the same bits.
+// Loads are whole 128-byte runs: the row pitch is a multiple of 32, so the last, ragged row block reads rows past
+// n_rows inside the pitch and never stores them.
+__global__ void __launch_bounds__(SBN_TRIPLE_MAX_THREADS, 1) sbn_triple_kernel(const __grid_constant__ SbnTripleParams p) {
+    constexpr int T = SBN_PAIR_T, R = SBN_TRIPLE_ROWS;
+    extern __shared__ __align__(128) float s_ring[];
+    sbn_pdl_entry();
+    const int G = p.group, NT = p.n_tiles, S = p.n_stages;
+    const int nA = G * T * T, nB = NT * T * T, nE = nA + 2 * nB;
+    const uint32_t ld = static_cast<uint32_t>(p.ld);
+    const int4 *const tiles = reinterpret_cast<const int4 *>(p.tile_off);
+    // element offset (scaled by the row pitch; fits 32 bits: sbn_pair_fits) of every staged entry, per p
+    uint32_t *const s_off = reinterpret_cast<uint32_t *>(s_ring + S * nE * R);
+    for (int i = threadIdx.x; i < T * nE; i += blockDim.x) {
+        const int pp = i / nE, e = i % nE;
+        int off;
+        if (e < nA) {
+            off = __ldg(tiles).y + pp * p.a_p + (e / (T * T)) * p.a_g + (e / T % T) * p.a_k + (e % T) * p.a_j;
+        } else if (e < nA + nB) {
+            const int f = e - nA;
+            off = __ldg(tiles + f / (T * T)).z + pp * p.b_p + (f / T % T) * p.b_j + (f % T) * p.b_s;
+        } else {
+            const int f = e - nA - nB;
+            off = __ldg(tiles + f / (T * T)).w + pp * p.c_p + (f / T % T) * p.c_k + (f % T) * p.c_z;
+        }
+        s_off[i] = static_cast<uint32_t>(off) * ld;
+    }
+    __syncthreads();
+
+    const int n_rb = (p.n_rows + R - 1) / R;
+    const int n_items = (n_rb - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x) * T;
+    auto issue = [&](int it) {
+        if (it < n_items) {
+            const uint32_t row0 = (blockIdx.x + static_cast<uint32_t>(it / T) * gridDim.x) * R;
+            const uint32_t *const off = s_off + (it % T) * nE;
+            float *const dst = s_ring + (it % S) * nE * R;
+#pragma unroll 4
+            for (int c = threadIdx.x; c < nE * 8; c += blockDim.x) {
+                const int e = c >> 3, q = (c & 7) * 4;
+                const float *const src = e < nA ? p.a : (e < nA + nB ? p.b : p.c);
+                triple_cp_async16(dst + e * R + q, src + (off[e] + row0 + q));
+            }
+        }
+        asm volatile("cp.async.commit_group;" ::: "memory");  // empty past the last item: the group count stays uniform
+    };
+
+    const int lane = threadIdx.x & 31, rp = lane & 15;
+    const int slot = 2 * (threadIdx.x >> 5) + (lane >> 4);
+    const bool active = slot < G * NT;
+    const int g = active ? slot % G : 0, t = active ? slot / G : 0;
+    const int sa = g * T * T * R + 2 * rp, sb = (nA + t * T * T) * R + 2 * rp, sc = (nA + nB + t * T * T) * R + 2 * rp;
+    float *const op = p.out + static_cast<uint32_t>(__ldg(tiles + t).x + g * p.o_g) * ld;
+    const uint32_t oz = static_cast<uint32_t>(p.o_z) * ld, os = static_cast<uint32_t>(p.o_s) * ld;
+
+    float acc[T][T][2];  // [z][s][row]
+#pragma unroll
+    for (int z = 0; z < T; ++z)
+#pragma unroll
+        for (int s = 0; s < T; ++s) acc[z][s][0] = acc[z][s][1] = 0.f;
+    for (int i = 0; i < S - 1; ++i) issue(i);
+#pragma unroll 1
+    for (int it = 0; it < n_items; ++it) {
+        triple_cp_async_wait(S - 2);  // this thread's copies of item `it` have landed ...
+        __syncthreads();              // ... everyone's, and every thread is done with item it - 1, whose stage is refilled now
+        issue(it + S - 1);
+        if (active) {
+            const float *const st = s_ring + (it % S) * nE * R;
+            float bv[T][T][2];  // B[j][s]
+#pragma unroll
+            for (int j = 0; j < T; ++j)
+#pragma unroll
+                for (int s = 0; s < T; ++s) sbn_ldv<2>(bv[j][s], st + sb + (j * T + s) * R);
+#pragma unroll
+            for (int k = 0; k < T; ++k) {
+                float n[T][2], a[2];  // N[k][s] = sum_j A[k][j] B[j][s]
+                sbn_ldv<2>(a, st + sa + k * T * R);
+#pragma unroll
+                for (int s = 0; s < T; ++s) triple_mul2(n[s], a, bv[0][s]);
+#pragma unroll
+                for (int j = 1; j < T; ++j) {
+                    sbn_ldv<2>(a, st + sa + (k * T + j) * R);
+#pragma unroll
+                    for (int s = 0; s < T; ++s) sbn_fma2(n[s], a, bv[j][s]);
+                }
+#pragma unroll
+                for (int z = 0; z < T; ++z) {
+                    float c[2];
+                    sbn_ldv<2>(c, st + sc + (k * T + z) * R);
+#pragma unroll
+                    for (int s = 0; s < T; ++s) sbn_fma2(acc[z][s], c, n[s]);
+                }
+            }
+        }
+        if (it % T == T - 1) {
+            const int b = (blockIdx.x + (it / T) * gridDim.x) * R + 2 * rp;
+            if (active && b < p.n_rows) {
+                float *const o = op + b;
+#pragma unroll
+                for (int z = 0; z < T; ++z)
+#pragma unroll
+                    for (int s = 0; s < T; ++s) {
+                        if (b + 1 < p.n_rows) sbn_stv<2>(o + (z * oz + s * os), acc[z][s]);
+                        else __stcs(o + (z * oz + s * os), acc[z][s][0]);
+                    }
+            }
+#pragma unroll
+            for (int z = 0; z < T; ++z)
+#pragma unroll
+                for (int s = 0; s < T; ++s) acc[z][s][0] = acc[z][s][1] = 0.f;
+        }
+    }
+}
+
+// staged body: p-slices in the shared-memory ring, CTA size (16 row pairs x the (group digit, tile) slots, two per
+// warp) and dynamic shared memory (the ring + the per-p entry offsets)
+int triple_stages() {
+    static const int v = [] {
+        const char *e = getenv("SOROBN_B200_TRIPLE_STAGES");
+        const int s = e ? atoi(e) : 3;
+        return std::min(std::max(s, 2), SBN_TRIPLE_MAX_STAGES);
+    }();
+    return v;
+}
+int triple_threads(const SbnTripleParams &q) { return 32 * ((q.group * q.n_tiles + 1) / 2); }
+int triple_entries(const SbnTripleParams &q) { return (q.group + 2 * q.n_tiles) * SBN_PAIR_T * SBN_PAIR_T; }
+int triple_smem(const SbnTripleParams &q) {
+    return triple_entries(q) * (q.n_stages * SBN_TRIPLE_ROWS + SBN_PAIR_T) * 4;
+}
+constexpr int kTripleSmemMax = SBN_TRIPLE_MAX_ENTRIES * (SBN_TRIPLE_MAX_STAGES * SBN_TRIPLE_ROWS + SBN_PAIR_T) * 4;
 
 void launch_modes(const SbnPair &pr, const SbnPairParams &q, unsigned grid, size_t smem, cudaStream_t stream) {
     const dim3 g(grid), b(SBN_PAIR_ROWS / kV);
@@ -573,14 +732,32 @@ SbnPair *plan_triple(sbn_program *P, int i1, int i2, std::vector<int32_t> *tiles
             dig[k] = 0;
         }
     }
+    // the staged body: A's entries must not depend on the tile (they are staged once for all tiles), and one p-slice
+    // of A, B and C must fit SBN_TRIPLE_MAX_ENTRIES
+    bool staged = (q.group + 2 * n_tiles) * T * T <= SBN_TRIPLE_MAX_ENTRIES;
+    for (int64_t t = 1; t < n_tiles && staged; ++t) staged = (*tiles)[pr->tile_off_pos + 4 * t + 1] == (*tiles)[pr->tile_off_pos + 1];
+    pr->staged_ctas = staged ? 1 : 0;  // the real count: triple_capacity
+    q.n_stages = triple_stages();
     return pr;
+}
+
+// CTAs of the staged body that are resident at once on P's device (its launches are one wave of them)
+cudaError_t triple_capacity(sbn_program *P, SbnPair *pr) {
+    int per_sm = 0, n_sm = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sbn_triple_kernel, triple_threads(pr->t),
+                                                                  triple_smem(pr->t));
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, P->device);
+    if (e == cudaSuccess && per_sm < 1) e = cudaErrorInvalidConfiguration;
+    pr->staged_ctas = per_sm * n_sm;
+    return e;
 }
 
 }  // namespace
 
 cudaError_t sbn_pair_set_attrs() {
-    // 40 KB of dynamic shared memory at most: below the 48 KB every kernel may use without opting in
-    return cudaSuccess;
+    // the pair kernel takes 40 KB of dynamic shared memory at most: below the 48 KB every kernel may use without
+    // opting in; the staged triple body's ring takes up to 195 KB
+    return cudaFuncSetAttribute(sbn_triple_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTripleSmemMax);
 }
 
 void sbn_pair_free(sbn_program *P) {
@@ -629,6 +806,7 @@ cudaError_t sbn_pair_plan(sbn_program *P) {
                 P->pair_first[i1] = static_cast<int>(P->pairs.size());
                 P->pair_first[i2] = -2;
                 P->pairs.push_back(tr);
+                if (tr->staged_ctas && (err = triple_capacity(P, tr)) != cudaSuccess) return err;
                 continue;
             }
         }
@@ -791,6 +969,16 @@ static cudaError_t triple_launch(sbn_program *P, const SbnPair &pr, int64_t n_ro
     q.ld = P->ld;
     q.n_rows = static_cast<int32_t>(n_rows);
     q.tile_off = P->d_pair_tiles + pr.tile_off_pos;
+    // SOROBN_B200_TRIPLE_KERNEL=0 selects the L1 body; read at every launch, so that one process can time both
+    const char *body = getenv("SOROBN_B200_TRIPLE_KERNEL");
+    if (pr.staged_ctas > 0 && !(body && atoi(body) == 0)) {
+        // one wave of CTAs, each walking row blocks: the ring stays full across row blocks
+        const int64_t n_rblocks = (n_rows + SBN_TRIPLE_ROWS - 1) / SBN_TRIPLE_ROWS;
+        const int64_t grid = std::min<int64_t>(n_rblocks, pr.staged_ctas);
+        sbn_launch(sbn_triple_kernel, dim3(static_cast<unsigned>(grid)), dim3(triple_threads(q)),
+                   static_cast<size_t>(triple_smem(q)), stream, q);
+        return cudaGetLastError();
+    }
     // with a group axis: 32 rows x T group digits per CTA; without: 128 rows
     const int rows_per_cta = q.group > 1 ? 32 : 128;
     const int64_t n_rblocks = (n_rows + rows_per_cta - 1) / rows_per_cta;
@@ -811,9 +999,9 @@ static cudaError_t triple_launch(sbn_program *P, const SbnPair &pr, int64_t n_ro
     const int64_t grid = q.n_chunks * n_rblocks;
     if (grid >= (1LL << 31)) return cudaErrorInvalidConfiguration;
     const dim3 g(static_cast<unsigned>(grid)), b(rows_per_cta, q.group);
-    if (minb == 3) sbn_launch(sbn_triple_kernel<3>, g, b, 0, stream, q);
-    else if (minb == 1) sbn_launch(sbn_triple_kernel<1>, g, b, 0, stream, q);
-    else sbn_launch(sbn_triple_kernel<2>, g, b, 0, stream, q);
+    if (minb == 3) sbn_launch(sbn_triple_kernel_l1<3>, g, b, 0, stream, q);
+    else if (minb == 1) sbn_launch(sbn_triple_kernel_l1<1>, g, b, 0, stream, q);
+    else sbn_launch(sbn_triple_kernel_l1<2>, g, b, 0, stream, q);
     return cudaGetLastError();
 }
 

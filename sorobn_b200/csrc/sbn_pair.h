@@ -84,8 +84,19 @@ enum SbnPairMode { SBN_PAIR_B = 0, SBN_PAIR_CU = 1, SBN_PAIR_CE = 2, SBN_PAIR_GB
 // all operands batched, no tables.  The 3125-entry intermediate costs 25,000 B per row to write and read back;
 // a thread that owns one row and one combination of the untouched axes (a.., q..) walks p, and per p computes
 // N[k][s] = sum_j A[k][j] B[j][s] and out[z][s] += sum_k C[k][z] N[k][s] from 75 loaded entries -- the
-// intermediate never exists.  The operands are re-read once per combination of the axes they lack (from L2: CTAs
-// that are resident together work on the same row blocks).
+// intermediate never exists.
+//
+// Two kernel bodies.  `sbn_triple_kernel` (the default) gives a CTA a block of 32 rows and every combination of the
+// untouched axes: per p it stages the 32-row runs of all A, B and C entries of that p in shared memory (cp.async, a
+// ring of `n_stages` p-slices), so each operand entry crosses HBM once per row; a thread then takes 2 rows (one
+// register pair, packed FFMA2) and one (group digit, tile), keeps its 25 entries of B in registers and walks k.  It
+// needs A to be the same for every tile and at most 15 x 25 entries per p (`SbnPair::staged_ctas`).
+// `sbn_triple_kernel_l1` (SOROBN_B200_TRIPLE_KERNEL=0, and every triple the staged body does not cover) is one row per
+// thread with the operands re-read once per combination of the axes they lack (from L1 / L2).
+#define SBN_TRIPLE_ROWS 32            // rows per block of the staged body: the row pitch is a multiple of it
+#define SBN_TRIPLE_MAX_ENTRIES 375    // operand entries staged per p: A (group x 25) + B and C (25 per tile each)
+#define SBN_TRIPLE_MAX_STAGES 4
+#define SBN_TRIPLE_MAX_THREADS 416    // 16 row pairs x 26 (group digit, tile) slots
 struct SbnTripleParams {
     const float *a, *b, *c;
     float *out;
@@ -99,6 +110,7 @@ struct SbnTripleParams {
     int32_t o_z, o_s;
     int32_t group;                // 1, or T: threadIdx.y walks the T digits of a tile axis only A carries ...
     int32_t a_g, o_g;             // ... with these entry strides in A and in the output
+    int32_t n_stages;             // staged body: p-slices in the shared-memory ring (2 .. SBN_TRIPLE_MAX_STAGES)
 };
 
 // One planned pair (host side).
@@ -111,6 +123,7 @@ struct SbnPair {
     SbnPairParams q;              // everything but the run-time pointers
     SbnTripleParams t;
     int a_in, b_in, c_in;         // kind 1: operand indices (A, B among step1's inputs, C among step2's)
+    int staged_ctas;              // kind 1: CTAs of the staged body that fit the device at once, 0 when it does not apply
     int64_t tile_off_pos;         // int32 offset into the pair tile table
     int64_t canon_pos;            // float offset into the canonical coefficient buffer
 };
